@@ -139,8 +139,44 @@ def usable_cores():
 
 PECAN_BYTES_PER_CELL = 120.0   # SURVEY.md 8d: 5 fp64 states x (forward write + forward read at the traceback + backward write)
 
+# --dump-outputs keeps every per-end / per-pair summary but the full alignments of a fixed sample only (64 MB in all at most)
+DUMP_SAMPLE_ENDS, DUMP_SAMPLE_PAIRS = 256, 64
 
-def pecan_measure(local_rank, rank, first_pair, n_pairs, steps, warmup, cpu_budget, want_cpu, no_e2e, host_threads):
+
+def _dump_sample(n, k):
+    """a fixed, seeded choice of min(n, k) of n indices, increasing"""
+    return np.sort(np.random.default_rng(0).choice(n, min(n, k), replace=False))
+
+
+def dump_poa_outputs(d, msas, cells):
+    """what the batched POA returned after the last timed step: every end's MSA width, banded cells and FNV-1a MSA hash (as
+    its two 32-bit halves, exact in float64), and the MSA bytes of a fixed sample of ends (each [K, width] matrix flattened,
+    concatenated in the order of poa_sample_ends)"""
+    os.makedirs(d, exist_ok=True)
+    idx = _dump_sample(len(msas), DUMP_SAMPLE_ENDS)
+    h = np.array([workload.msa_hash(m) for m in msas], np.uint64)
+    np.save(os.path.join(d, "poa_msa_columns.npy"), np.array([m.shape[1] for m in msas], np.float64))
+    np.save(os.path.join(d, "poa_cells.npy"), np.asarray(cells, np.float64))
+    np.save(os.path.join(d, "poa_msa_hash.npy"), np.stack([h >> np.uint64(32), h & np.uint64(0xffffffff)], 1).astype(np.float64))
+    np.save(os.path.join(d, "poa_sample_ends.npy"), idx.astype(np.float64))
+    np.save(os.path.join(d, "poa_sample_msa.npy"), np.concatenate([msas[i].reshape(-1) for i in idx]).astype(np.float32))
+
+
+def dump_pecan_outputs(d, res):
+    """what the pair-HMM stage returned after the last timed step: every pair's triple count, banded cells and sum of integer
+    scores, and the (score, x, y) triples and pre-floor posteriors of a fixed sample of pairs (concatenated in the order of
+    pecan_sample_pairs)"""
+    os.makedirs(d, exist_ok=True)
+    idx = _dump_sample(len(res), DUMP_SAMPLE_PAIRS)
+    np.save(os.path.join(d, "pecan_triples_per_pair.npy"), np.array([len(r[0]) for r in res], np.float64))
+    np.save(os.path.join(d, "pecan_cells.npy"), np.array([r[2] for r in res], np.float64))
+    np.save(os.path.join(d, "pecan_score_sums.npy"), np.array([r[0][:, 0].sum() for r in res], np.float64))
+    np.save(os.path.join(d, "pecan_sample_pairs.npy"), idx.astype(np.float64))
+    np.save(os.path.join(d, "pecan_sample_triples.npy"), np.concatenate([res[i][0] for i in idx]).reshape(-1, 3).astype(np.float64))
+    np.save(os.path.join(d, "pecan_sample_posteriors.npy"), np.concatenate([res[i][1] for i in idx]).astype(np.float64))
+
+
+def pecan_measure(local_rank, rank, first_pair, n_pairs, steps, warmup, cpu_budget, want_cpu, no_e2e, host_threads, dump_dir=None):
     """cPecan mode (SURVEY.md 8a row a13, BASELINE.json configs[3]): banded pair-HMM posteriors of n_pairs synthetic
     2 kbp pairs per GPU per step with MUM-like anchors (k = 50, Cactus' setting). Runs in a process of its own (see main)
     and returns this rank's raw measurements."""
@@ -156,6 +192,8 @@ def pecan_measure(local_rank, rank, first_pair, n_pairs, steps, warmup, cpu_budg
         dev_ms += st.run()             # CUDA-event time of the launch(es); the call returns after the stream is idle
         launches += st.launches()
     res = st.fetch(True)
+    if dump_dir:
+        dump_pecan_outputs(dump_dir, res)
     n_trip = int(sum(len(r[0]) for r in res))
     st.close()
     out = {"dev_ms": dev_ms, "launches": launches, "cells": cells, "n_pairs": n_pairs, "steps": steps, "e2e_ms": float("nan"), "same": True,
@@ -570,6 +608,8 @@ def gpu_arm(args):
     barrier()
     wall_ms = (time.time() - t0) * 1e3
     msas, cells = stage.fetch()
+    if args.dump_outputs and rank == 0:
+        dump_poa_outputs(args.dump_outputs, msas, cells)
     my_cells = float(cells.sum())
     buckets = stage.buckets()
 
@@ -714,6 +754,7 @@ def gpu_arm(args):
                "--steps", str(args.steps), "--warmup", str(args.warmup), "--cpu-budget", str(args.cpu_budget)]
         cmd += ["--no-e2e"] if args.no_e2e else []
         cmd += ["--no-cpu-baseline"] if args.no_cpu_baseline else []
+        cmd += ["--dump-outputs", args.dump_outputs] if args.dump_outputs and rank == 0 else []
         env = dict(os.environ)
         env["OMP_NUM_THREADS"] = str(host_threads)
         barrier()
@@ -803,7 +844,12 @@ def main():
     ap.add_argument("--pecan-only", action="store_true", help="internal: this process only measures the cPecan section and prints its raw numbers")
     ap.add_argument("--pecan-pairs-per-step", type=int, default=int(os.environ.get("BARB200_PECAN_PAIRS_PER_STEP", "4736")),
                     help="cPecan-mode pairs per GPU per step (default 32 x 148 SMs); 0 skips the cPecan section")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed POA and cPecan steps returned in their last step as DIR/<name>.npy (float32 / float64; "
+                         "per-end and per-pair summaries of the whole step, full alignments of a fixed sample); GPU arm, rank 0")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     if args.flowers_only:
         import cactus_b200 as cb
@@ -816,8 +862,8 @@ def main():
         world = int(os.environ.get("WORLD_SIZE", "1"))
         local_rank = int(os.environ.get("LOCAL_RANK", "0"))
         host_threads = int(os.environ.get("OMP_NUM_THREADS", "0")) or max(1, usable_cores() // max(1, int(os.environ.get("LOCAL_WORLD_SIZE", str(world)))))
-        m = pecan_measure(local_rank, rank, rank * args.pecan_pairs_per_step, args.pecan_pairs_per_step, max(1, min(args.steps, 3)),
-                          max(1, min(args.warmup, 2)), min(args.cpu_budget, 12.0), not args.no_cpu_baseline, args.no_e2e, host_threads)
+        m = pecan_measure(local_rank, rank, rank * args.pecan_pairs_per_step, args.pecan_pairs_per_step, args.steps, args.warmup,
+                          min(args.cpu_budget, 12.0), not args.no_cpu_baseline, args.no_e2e, host_threads, args.dump_outputs)
         print("PECAN_JSON " + json.dumps(m))
         return 0
     if args.impl == "reference":

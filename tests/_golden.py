@@ -1,10 +1,50 @@
 """Readers for the committed golden vectors (tests/golden/*.npz, produced from the unmodified reference by
-scripts/make_golden.py)."""
+scripts/make_golden.py) and for the reference's output digests of the seeded differential tests (tests/golden/ref_digests.json,
+scripts/make_golden_ref_digests.py)."""
+import hashlib
+import json
 import os
 
 import numpy as np
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REF_DIGESTS = os.path.join(GOLD, "ref_digests.json")
+
+
+def digest(*arrays):
+    """sha256 (first 16 hex digits) over the dtype, shape and bytes of each array"""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(repr((a.dtype.str, a.shape)).encode())
+        h.update(a.tobytes())
+    return h.hexdigest()[:16]
+
+
+def trace_digest(tr):
+    """the fields of an _reflib trace that the differential tests compare, reduced to digests and scalars"""
+    alns = tr["alns"]
+    return {"msa_len": int(tr["msa_len"]), "cells": int(tr["cells"]), "msa": digest(tr["msa"]),
+            "order": digest(np.array(tr["read_id_map"], np.int64)),
+            "alns": digest(np.array([[a["read_id"], a["qlen"], a["node_n"], a["best_score"]] for a in alns], np.int64).reshape(-1, 4)),
+            "cigar": digest(*[a["cigar"] for a in alns]),
+            "dp": digest(*[np.concatenate([a["dp_beg"], a["dp_end"]]) for a in alns])}
+
+
+_ref_digests = None
+
+
+def check_ref_digest(key, inputs, out):
+    """`out` (a dict of digests and scalars) must equal what the unmodified reference produced for the case `key`, whose
+    inputs had the digest `inputs`"""
+    global _ref_digests
+    if _ref_digests is None:
+        with open(REF_DIGESTS) as f:
+            _ref_digests = json.load(f)
+    want = _ref_digests[key]
+    assert inputs == want["in"], "%s: the inputs are not the ones the reference's digests were made from" % key
+    diff = {k: (out.get(k), want["out"].get(k)) for k in set(out) | set(want["out"]) if out.get(k) != want["out"].get(k)}
+    assert not diff, "%s differs from the reference (got, want): %s" % (key, diff)
 
 
 def poa_cases():

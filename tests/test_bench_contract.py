@@ -12,7 +12,7 @@ import _reflib as R
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not (R.have_ref() and R.have_pecan_ref()), reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(not (R.have_ref() and R.have_pecan_ref()), reason="oracle/_ref not built (needs the reference's sources, see oracle/Makefile)")
 def test_reference_arm_prints_one_json_line():
     cp = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
                          "--cpu-budget", "1", "--ends-per-step", "8", "--pecan-pairs-per-step", "8"],

@@ -19,7 +19,7 @@ def test_random_flower_is_deterministic():
     assert a["seqs"] == b["seqs"] and a["adj"] == b["adj"]
 
 
-@pytest.mark.skipif(not F.have("ref"), reason="oracle/_ref/libflower_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not F.have("ref"), reason="oracle/_ref/libflower_ref.so not built (needs the reference's sources, see oracle/Makefile)")
 def test_reference_library_reproduces_the_fixture():
     for name, fl, params, stream, bar in G.cases():
         r = F.blocks("ref", fl, params)
@@ -30,7 +30,7 @@ def test_reference_library_reproduces_the_fixture():
         assert np.array_equal(o, c[4]), c[0]
 
 
-@pytest.mark.skipif(not F.have("standin"), reason="oracle/_ref/libflower_standin.so not built (needs /root/reference)")
+@pytest.mark.skipif(not F.have("standin"), reason="oracle/_ref/libflower_standin.so not built (needs the reference's sources, see oracle/Makefile)")
 def test_shims_and_host_code_over_a_standin_device_reproduce_the_fixture():
     """no GPU: the REAL shims (shim/cactus_bar_shim.c incl. its bar()) and the REAL host code of the product (host_bar.cpp,
     end_queue.h, bar_windows.h) under the reference's own flower-level objects, with a TEST-ONLY CPU stand-in for the device
@@ -47,7 +47,7 @@ def test_shims_and_host_code_over_a_standin_device_reproduce_the_fixture():
         assert np.array_equal(a, b), i
 
 
-@pytest.mark.skipif(not (F.have("harvest") and F.have("standin")), reason="oracle/_ref/libflower_harvest.so not built (needs /root/reference)")
+@pytest.mark.skipif(not (F.have("harvest") and F.have("standin")), reason="oracle/_ref/libflower_harvest.so not built (needs the reference's sources, see oracle/Makefile)")
 def test_harvested_inputs_replay_to_the_same_alignments(tmp_path, oracle_built):
     """shim/cactus_bar_harvest.c records the inputs of every top-level alignment call of a REFERENCE bar() run (the way real
     datasets are to be captured for bench.py --workload); replaying the record through the product's host code (stand-in
@@ -87,7 +87,7 @@ def pecan_flowers():
            [F.random_flower(500 + s, n_threads=14 + s, n_blocks=2, seg_len=70, p_skip=0.0, p_loop=0.0) for s in range(2)]
 
 
-@pytest.mark.skipif(not F.have("standin"), reason="oracle/_ref/libflower_standin.so not built (needs /root/reference)")
+@pytest.mark.skipif(not F.have("standin"), reason="oracle/_ref/libflower_standin.so not built (needs the reference's sources, see oracle/Makefile)")
 def test_cpecan_configuration_through_the_pecan_shim_on_the_standin_device():
     """bar() with partialOrderAlignment="0": the reference's makeFlowerAlignment3 / makeEndAlignment / poset code over
     shim/cactus_pecan_shim.c (makeAlignment with every selection round as one device batch, makeAllPairwiseAlignments,

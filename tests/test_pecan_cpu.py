@@ -50,18 +50,26 @@ def test_reference_known_answer(oracle_built):
     assert {(int(x), int(y)) for _, x, y in t} == want
 
 
-@pytest.mark.skipif(not R.have_pecan_ref(), reason="oracle/_ref/libpecan_ref.so not built (needs /root/reference)")
-def test_oracle_vs_reference_random(oracle_built):
+def random_reference_cases():
+    """the seeded cases of test_oracle_vs_reference_random: (key, inputs digest, case, whether the posteriors of its single
+    sub-matrix are compared too)"""
     rng = np.random.default_rng(4242)
     for it in range(60):
         sx, sy, a, rl, rr, p, sb = _random_case(rng)
-        tr = R.ref_pecan_aligned_pairs(sx, sy, a, rl, rr, p, sb)
-        to, po = R.oracle_pecan_aligned_pairs(sx, sy, a, rl, rr, p, sb)
-        assert np.array_equal(tr, to), (it, len(sx), len(sy), len(a))
-        if len(R.oracle_pecan_split_points(len(sx), len(sy), a, sb, rl, rr)) == 1:
-            x, y, ps = R.ref_pecan_posteriors(sx, sy, a, rl, rr, p)
-            xo, yo, pso = R.oracle_pecan_posteriors(sx, sy, a, rl, rr, p)
-            assert np.array_equal(x, xo) and np.array_equal(y, yo) and np.array_equal(ps, pso), it
+        inputs = G.digest(np.frombuffer(sx, np.uint8), np.frombuffer(sy, np.uint8), np.asarray(a, np.int64).reshape(-1, 2),
+                          np.array([rl, rr, sb], np.int64), np.frombuffer(bytes(p), np.uint8))
+        single = len(R.oracle_pecan_split_points(len(sx), len(sy), a, sb, rl, rr)) == 1
+        yield "pecan_random/%d" % it, inputs, (sx, sy, a, rl, rr, p, sb), single
+
+
+def test_oracle_vs_reference_random(oracle_built):
+    """the oracle's triples (and, for a single sub-matrix, its pre-floor posteriors) against the unmodified reference's, stored as
+    digests in tests/golden/ref_digests.json (scripts/make_golden_ref_digests.py)"""
+    for key, inputs, (sx, sy, a, rl, rr, p, sb), single in random_reference_cases():
+        out = {"triples": G.digest(R.oracle_pecan_aligned_pairs(sx, sy, a, rl, rr, p, sb)[0])}
+        if single:
+            out["posteriors"] = G.digest(*R.oracle_pecan_posteriors(sx, sy, a, rl, rr, p))
+        G.check_ref_digest(key, inputs, out)
 
 
 def test_warp_program_golden():
